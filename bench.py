@@ -2,6 +2,7 @@
 """bench.py -- WSI tiles/sec through the RoI stage + merge (BASELINE.json metric) on N B200s of one node.
 
     python bench.py --gpus 1 --steps 20 --warmup 3                      # our arm
+    python bench.py --gpus 1 --steps 20 --warmup 3 --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
     python bench.py --impl reference --gpus 1 --steps 2 --warmup 1      # reference CPU path (oracle port)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
@@ -63,7 +64,13 @@ def parse():
     p.add_argument("--inflight", type=int, default=3, help="batches in flight: consecutive steps alternate between this many "
                    "streams (each with its own captured graph), so the latency-bound tail of one batch (NMS scans, mask NMS, "
                    "contours) overlaps the RoIAlign of the next; 1 = strictly one step after another")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write the RoI-stage result of the last step and the merge's kept nuclei as "
+                        "DIR/<name>.npy (rank 0), to compare two builds output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
 
 
 def stage_config(args):
@@ -419,6 +426,9 @@ def run_ours(args):
         dist.all_gather(tl, torch.tensor([steps_ms], device=dev, dtype=torch.float64))
         per_rank_steps = [float(t.item()) for t in tl]
     launches = _lib.LAUNCHES["n"] + (launches_per_step * args.steps if graph is not None else 0)
+    if args.dump_outputs and rank == 0:
+        last = res if graph is None else graph_res[(args.steps - 1) % len(graphs)]
+        dump_outputs(args.dump_outputs, last, kept)
 
     # ---- per-kernel durations (CUDA events cannot bracket nodes inside a graph): the same K steps are repeated eagerly
     # with an event pair around every op; these feed `roofline`, `roofline_other` and `breakdown_ms_per_step` only
@@ -535,6 +545,44 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, res, kept, big_cap=24 << 20):
+    """What the timed path hands its caller, as out_dir/<name>.npy: the RoI-stage result of one step with the padding slots
+    dropped (RoIStageResult.compact()) and the merge's kept nuclei.  Integers become float32 (float64 when they are int64);
+    contour points past a detection's count are zeroed (unwritten).  The two per-detection arrays that can be large, dense
+    masks and contours, are limited to `big_cap` bytes each by a seeded row sample (the same rows for every build when the
+    detection count agrees); `*_rows` names the rows kept."""
+    os.makedirs(out_dir, exist_ok=True)
+    r = res.compact()
+    n = int(r.det_boxes.shape[0])
+    perm = torch.randperm(n, generator=torch.Generator().manual_seed(0))
+
+    def rows(row_bytes):
+        return perm[: min(n, big_cap // row_bytes)].sort().values
+
+    H, words = r.mask_bits.shape[1:]
+    mrows = rows(H * words * 64 * 4)
+    if r.masks is not None:
+        masks = r.masks[mrows.to(r.masks.device)]
+    else:                                                   # bit rows only: bit x % 64 of word x // 64 is pixel x
+        bits = r.mask_bits[mrows.to(r.mask_bits.device)]
+        masks = ((bits.unsqueeze(-1) >> torch.arange(64, device=bits.device)) & 1).flatten(-2).to(torch.uint8)
+    out = {"det_boxes": r.det_boxes, "det_scores": r.det_scores, "det_labels": r.det_labels, "det_tile": r.det_tile,
+           "det_cand": r.det_cand, "mask_area": r.mask_area, "keep": r.keep, "tile_start": r.tile_start,
+           "tile_count": r.tile_count, "masks_sample": masks, "masks_sample_rows": mrows, "merge_kept": kept}
+    if r.contour_xy is not None:
+        xy, cnt = r.contour_xy, r.contour_count
+        xy = xy * (torch.arange(xy.shape[1], device=xy.device)[None, :] < cnt[:, None]).unsqueeze(-1).to(xy.dtype)
+        crows = rows(xy.shape[1] * 2 * 4)
+        out.update(contour_count=cnt, contour_xy_sample=xy[crows.to(xy.device)], contour_xy_sample_rows=crows)
+    for name, t in out.items():
+        if t is None:
+            continue
+        a = t.detach().cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64 if a.dtype == np.int64 else np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class NucleiAccumulator:

@@ -3,6 +3,7 @@ package never touches the oracle; ops refuse CPU tensors (no silent fallback).""
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 
 import pytest
@@ -31,9 +32,12 @@ def test_library_exports_every_declared_symbol():
 
 def test_library_is_sm100a_native():
     from nuhtc_b200 import _lib
-    out = subprocess.run(["cuobjdump", "--list-elf", _lib.LIB_PATH], capture_output=True, text=True)
-    if out.returncode != 0:
+    nvcc = shutil.which("nvcc")         # the toolkit that built the library
+    tool = shutil.which("cuobjdump") or (nvcc and shutil.which("cuobjdump", path=os.path.dirname(nvcc)))
+    if not tool:
         pytest.skip("cuobjdump unavailable")
+    out = subprocess.run([tool, "--list-elf", _lib.LIB_PATH], capture_output=True, text=True)
+    assert out.returncode == 0, out.stderr
     assert "sm_100a" in out.stdout
 
 

@@ -36,9 +36,14 @@ def test_fused_bbox_features_match_reference_bbox_forward():
     st = RoIStage(cfg, [None] * 3, None)
     rois = bbox2roi([p[:, :4] for p in plist]).cuda()
     out = st.extract(stage_levels([f.cuda() for f in feats]), rois, 7, 2, stage_levels([sem_feat.cuda()]), "bbox").cpu()
+    assert out.shape == (rois.shape[0], T.C, 7, 7)
+    # the golden keeps every k-th channel whole and, for every channel, the sum over the 7x7 bins
+    sums = out.double().sum((2, 3))
+    out = out[:, ::int(z["channel_stride"])]
     ref = torch.from_numpy(z["bbox_feats"])
     assert out.shape == ref.shape
     assert (out - ref).abs().max().item() <= 5e-5      # five summed terms (2 RoIAlign levels, 2 attention levels, semantic)
+    assert (sums - torch.from_numpy(z["bbox_feats_bin_sum"]).double()).abs().max().item() <= 49 * 5e-5
 
 
 def test_simple_test_matches_reference(oracle):

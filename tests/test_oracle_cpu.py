@@ -364,7 +364,10 @@ def test_golden_attention_extractor(oracle):
     z = np.load(os.path.join(G, "attention_extractor.npz"))
     feats = synth.fpn_levels(2, 64, frame=256, seed=21)
     out = oracle.attention_roi_extract(feats, torch.from_numpy(z["rois"]), (4, 8, 16, 32), 7, 2, start_level=2, thres=0.0)
-    assert torch.equal(out, torch.from_numpy(z["out"]))
+    assert out.shape == (z["rois"].shape[0], 64, 7, 7)
+    # the golden keeps every k-th channel whole and, for every channel, the sum over the 7x7 bins
+    assert torch.equal(out[:, ::int(z["channel_stride"])], torch.from_numpy(z["out"]))
+    assert torch.allclose(out.double().sum((2, 3)), torch.from_numpy(z["out_bin_sum"]).double(), rtol=1e-6, atol=1e-6)
 
 
 def test_rpn_post_process_golden(oracle):
