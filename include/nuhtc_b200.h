@@ -309,6 +309,18 @@ size_t nuhtc_mask_components_workspace_bytes(int B, int H, int W);
 int nuhtc_mask_components(const float *mask, int B, int H, int W, int min_area, int max_area, int max_boxes,
                           float *boxes, int32_t *counts, uint8_t *filled, void *ws, size_t ws_bytes, void *stream);
 
+/* ---- test-time image pipeline (SURVEY 8f-4, the tile loader) ---------------------------------
+ * Replaces the per-tile CPU work of `inference_detector(model, [np.ndarray]*B)` (tools/infer_wsi.py:485 ->
+ * mmdet/apis/inference.py:90-153) under the NuHTC test pipeline: Resize(keep_ratio=True) with cv2 INTER_LINEAR,
+ * Normalize(mean, std, to_rgb), Pad(size_divisor), ImageToTensor and the batch collate, in ONE launch.
+ *   tiles [B,h,w,3] uint8 HWC (device), out [B,3,pad_h,pad_w] fp32 (device, fully overwritten): the resized image in
+ *   [0,new_h) x [0,new_w), 0 elsewhere.  mean3 / std3: 3 HOST floats per OUTPUT channel (Normalize's float32 arrays);
+ *   to_rgb != 0 swaps channels 0 and 2.  Bit-exact with cv2.resize (uint8 fixed-point path) and with mmcv.imnormalize_
+ *   (cv2.subtract / cv2.multiply with float64 scalars).  Upscaling and identity only: new_h >= h, new_w >= w,
+ *   pad_h >= new_h, pad_w >= new_w.  B = 0 returns 0.  No allocation or synchronisation: CUDA-graph capturable. */
+int nuhtc_preprocess_tiles(const uint8_t *tiles, int B, int h, int w, int new_h, int new_w, int pad_h, int pad_w, int to_rgb,
+                           const float *mean3, const float *std3, float *out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

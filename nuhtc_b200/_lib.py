@@ -60,6 +60,7 @@ SIGNATURES = {
     "nuhtc_mask_components": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _c.c_size_t, _vp]),
     "nuhtc_ring_yextent": (_i, [_vp, _vp, _i64, _vp, _vp, _vp]),
     "nuhtc_keep_flags": (_i, [_vp, _vp, _vp, _i, _i, _i64, _vp, _vp]),
+    "nuhtc_preprocess_tiles": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _c.POINTER(_f * 3), _c.POINTER(_f * 3), _vp, _vp]),
 }
 
 _lib = None
@@ -108,7 +109,7 @@ def require_cuda(t: torch.Tensor, name: str) -> None:
 # ---- launch accounting: how many of OUR kernels each C-ABI call enqueues (bench.py reports the sum as
 # "gpu_launches"; library kernels such as cub's radix sort are not counted)
 LAUNCHES = {"n": 0}
-KERNELS_PER_CALL = {"nchw_to_nhwc": 1, "to_cg32": 1, "roi_align_strip": 5, "attention_pool": 4, "roi_align": 1, "nms": 9, "paste": 2, "paste_dual": 1, "pack": 3, "mask_nms": 8, "merge": 16, "contours": 2, "rings": 1, "glue": 1, "rpn_topk": 1, "components": 8}
+KERNELS_PER_CALL = {"nchw_to_nhwc": 1, "to_cg32": 1, "roi_align_strip": 5, "attention_pool": 4, "roi_align": 1, "nms": 9, "paste": 2, "paste_dual": 1, "pack": 3, "mask_nms": 8, "merge": 16, "contours": 2, "rings": 1, "glue": 1, "rpn_topk": 1, "components": 8, "preprocess": 1}
 
 
 def count(op: str, n: int = 1) -> None:

@@ -55,3 +55,11 @@ def patch_wsi_tools(infer_wsi_module=None, nuclei_merge_module=None):
         nuclei_merge_module.merge_overlap = merge_overlap
         done.append("nuclei_merge.merge_overlap")
     return done
+
+
+def patch_inference(infer_wsi_module):
+    """Rebind ``inference_detector`` of tools/infer_wsi.py (called at :485) to :func:`nuhtc_b200.inference_detector`: the
+    tiles' resize / normalise / pad run as one kernel on the GPU and cross PCIe as uint8.  Pass the imported module."""
+    from . import inference_detector
+    infer_wsi_module.inference_detector = inference_detector
+    return ["infer_wsi.inference_detector"]

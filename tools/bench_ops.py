@@ -157,6 +157,16 @@ def main():
         ms, best = timeit(lambda: ws.mask_components(m))
         bx, cnt = ws.mask_components(m)
         rec("watershed_components_16x512", ms, best, B * 512 * 512 * 5, instances=int(cnt.sum().item()))
+    if want("preprocess"):
+        # one TilePipeline call from a uint8 CUDA tensor, host overhead included; the output block is reused from call to
+        # call, so tools/bench_preprocess.py is where the kernel is timed with an L2-exceeding working set
+        from nuhtc_b200.preprocess import TilePipeline
+        t = torch.randint(0, 256, (B, 256, 256, 3), dtype=torch.uint8, device=dev, generator=torch.Generator(device=dev).manual_seed(0))
+        for s in (2.0, 4.0):
+            pipe = TilePipeline(s, [123.675, 116.28, 103.53], [58.395, 57.12, 57.375])
+            ph, pw = pipe.sizes(256, 256)[2:4]
+            ms, best = timeit(lambda: pipe(t))
+            rec(f"preprocess_{B}x256_to_{ph}", ms, best, t.numel() + B * 3 * ph * pw * 4)
     if want("merge"):
         d = synth.slide_nuclei(64, 64, per_tile=23, seed=0)
         xy, voff, sc = (torch.from_numpy(d[k]).to(dev) for k in ("xy", "voff", "score"))
