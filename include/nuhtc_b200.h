@@ -91,6 +91,22 @@ int nuhtc_roi_align_cg32(const float *const *feats, const int *H, const int *W, 
                          float finest_scale, const int *pool2, float *out, const float *bias, void *ws, size_t ws_bytes,
                          void *stream);
 
+/* ---- half-precision levels and RoI features ---------------------------------------------------------------------
+ * mmcv's force_fp32(out_fp16=True) contract, extended to bf16.  nuhtc_to_cg32_dt stages fp32, fp16 or bf16 levels
+ * (in_dtype) into the same fp32 CG32 buffer: the upcast is exact, so the staged bytes equal those of the fp32 level.
+ * nuhtc_roi_align_cg32_dt computes exactly what nuhtc_roi_align_cg32 computes, in fp32 (bias stays fp32), and rounds
+ * every output value once, round-to-nearest-even, to out_dtype.  `in` must be aligned to 4 elements of in_dtype and
+ * `out` to 16 bytes; an unknown dtype code or a misaligned pointer returns NUHTC_EINVAL before any CUDA call.
+ * nuhtc_to_cg32 / nuhtc_roi_align_cg32 are these calls with NUHTC_DTYPE_F32. */
+#define NUHTC_DTYPE_F32 0
+#define NUHTC_DTYPE_F16 1
+#define NUHTC_DTYPE_BF16 2
+int nuhtc_to_cg32_dt(const void *in, int in_dtype, float *out, int B, int C, int H, int W, int channels_last, void *stream);
+int nuhtc_roi_align_cg32_dt(const float *const *feats, const int *H, const int *W, const float *scale, int L, int B, int C,
+                            const float *rois, int K, int PH, int PW, int sampling_ratio, int aligned, int mode,
+                            float finest_scale, const int *pool2, void *out, int out_dtype, const float *bias, void *ws,
+                            size_t ws_bytes, void *stream);
+
 /* ---- cosine-attention pooling (AttentionRoIExtractor, levels >= start_level) ---------------------------------------
  * Replaces nuhtc/models/roi_extractors_cus.py:220-238 for one level: for RoI k with centre cell
  * (b, floor((y1+y2)/(2*stride)), floor((x1+x2)/(2*stride))) (clamped to the map),

@@ -19,6 +19,7 @@ ROI_ROUTE, ROI_SUM = 0, 1
 IMPL_AUTO, IMPL_DIRECT = 0, 1
 NMS_AGNOSTIC, NMS_OFFSET, NMS_PERCLASS, NMS_PERCLASS_RAW = 0, 1, 2, 3
 PASTE_PROB, PASTE_BIN, PASTE_BITS = 0, 1, 2
+DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 MAX_LEVELS = 8
 
 _c = ctypes
@@ -35,6 +36,9 @@ SIGNATURES = {
     "nuhtc_roi_align_workspace_bytes": (_sz, [_c.POINTER(_i), _c.POINTER(_i), _i, _i, _i, _i, _i]),
     "nuhtc_roi_align_cg32": (_i, [_c.POINTER(_vp), _c.POINTER(_i), _c.POINTER(_i), _c.POINTER(_f), _i, _i, _i, _vp, _i, _i, _i, _i,
                                   _i, _i, _f, _c.POINTER(_i), _vp, _vp, _vp, _sz, _vp]),
+    "nuhtc_to_cg32_dt": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp]),
+    "nuhtc_roi_align_cg32_dt": (_i, [_c.POINTER(_vp), _c.POINTER(_i), _c.POINTER(_i), _c.POINTER(_f), _i, _i, _i, _vp, _i, _i, _i,
+                                     _i, _i, _i, _f, _c.POINTER(_i), _vp, _i, _vp, _vp, _sz, _vp]),
     "nuhtc_attention_pool_workspace_bytes": (_sz, [_i, _i]),
     "nuhtc_attention_pool": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _f, _f, _i, _vp, _vp, _vp, _sz, _vp]),
     "nuhtc_nms_workspace_bytes": (_sz, [_i64, _i, _i64, _i]),
@@ -99,6 +103,10 @@ def stream_ptr(device=None) -> int:
 
 def ptr(t) -> int:
     return 0 if t is None else t.data_ptr()
+
+
+# element types the RoIAlign path takes natively (include/nuhtc_b200.h NUHTC_DTYPE_*)
+DTYPE_CODES = {torch.float32: DTYPE_F32, torch.float16: DTYPE_F16, torch.bfloat16: DTYPE_BF16}
 
 
 def require_cuda(t: torch.Tensor, name: str) -> None:

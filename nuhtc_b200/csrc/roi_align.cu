@@ -162,10 +162,11 @@ __device__ __forceinline__ void sweep_rows(const float *__restrict__ rowp, size_
 
 // P output size; NQ channel quads per VEC slice; PHS: the P output rows are split over PHS thread groups;
 // VEC: float4 slices per thread (a thread owns channels 4q..4q+3 of each slice).  CTA = (RoI, CC channels).
-template <int P, int NQ, int PHS, int VEC, int MINB>
+// OutT: output element type; the tile stays fp32 and every value is rounded once on its way out.
+template <int P, int NQ, int PHS, int VEC, int MINB, typename OutT>
 __global__ void __launch_bounds__(NQ *P *PHS, MINB) roi_align_sep_kernel(RoiLevels lv, int C, const float *__restrict__ rois, int sr,
                                                                     int aligned, int mode, float finest,
-                                                                    float *__restrict__ out, const float *__restrict__ bias,
+                                                                    OutT *__restrict__ out, const float *__restrict__ bias,
                                                                     int cg32, const int *__restrict__ list,
                                                                     const int *__restrict__ list_count) {
     constexpr int CC = NQ * 4 * VEC;
@@ -329,7 +330,7 @@ __global__ void __launch_bounds__(NQ *P *PHS, MINB) roi_align_sep_kernel(RoiLeve
         }
     }
     __syncthreads();
-    float *outp = out + ((size_t)k * C + c0) * PP;
+    OutT *outp = out + ((size_t)k * C + c0) * PP;
     constexpr int N4 = CC * PP / 4;
     for (int i = tid; i < N4; i += NT) {
         float4 v;
@@ -348,7 +349,7 @@ __global__ void __launch_bounds__(NQ *P *PHS, MINB) roi_align_sep_kernel(RoiLeve
             }
             v = make_float4(t[0], t[1], t[2], t[3]);
         }
-        st_stream_f4(outp + 4 * i, v);
+        st_stream4(outp + 4 * i, to_out<OutT>(v.x), to_out<OutT>(v.y), to_out<OutT>(v.z), to_out<OutT>(v.w));
     }
     }   // item loop
 }
@@ -358,21 +359,21 @@ static size_t sep_smem_bytes() {
     return sizeof(float) * (NQ * 4 * VEC * SepCfg<P>::S + 2 * P * kMaxTap) + sizeof(int) * (4 * P + 4);
 }
 
-template <int P, int NQ, int PHS, int VEC, int MINB>
+template <int P, int NQ, int PHS, int VEC, int MINB, typename OutT>
 static int launch_sep(const RoiLevels &lv, int C, const float *rois, int K, int sr, int aligned, int mode, float finest,
-                      float *out, const float *bias, cudaStream_t st, int cg32 = 0, const int *list = nullptr,
+                      OutT *out, const float *bias, cudaStream_t st, int cg32 = 0, const int *list = nullptr,
                       const int *list_count = nullptr) {
     static bool attr_done[kNuhtcMaxDevices] = {false};
     const int dev = nuhtc_device();
     const size_t smem = sep_smem_bytes<P, NQ, VEC>();
     if (!attr_done[dev]) {
-        NUHTC_CUDA(cudaFuncSetAttribute(roi_align_sep_kernel<P, NQ, PHS, VEC, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        NUHTC_CUDA(cudaFuncSetAttribute(roi_align_sep_kernel<P, NQ, PHS, VEC, MINB, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done[dev] = true;
     }
     // every RoI: one CTA each; a RoI list: a resident grid that walks the list (its length is only known on the device)
     const int gx = list ? (K < 4 * nuhtc_sm_count() ? K : 4 * nuhtc_sm_count()) : K;
     dim3 grid(gx, C / (NQ * 4 * VEC));
-    roi_align_sep_kernel<P, NQ, PHS, VEC, MINB><<<grid, NQ * P * PHS, smem, st>>>(lv, C, rois, sr, aligned, mode, finest, out, bias,
+    roi_align_sep_kernel<P, NQ, PHS, VEC, MINB, OutT><<<grid, NQ * P * PHS, smem, st>>>(lv, C, rois, sr, aligned, mode, finest, out, bias,
                                                                                   cg32, list, list_count);
     NUHTC_LAUNCH_CHECK();
     return NUHTC_OK;
@@ -486,10 +487,11 @@ __device__ __forceinline__ void staged_rows(const float *ring, int stage_floats,
 }
 
 // Warp roles: [0, NCONS) consumers, warp NCONS/32 builds tap tables (kPipeSlots items ahead), warp NCONS/32+1 streams rows.
-template <int P, int NQ, int PHS, int NS, int WMAX, int MINB>
+// OutT: output element type; values are rounded to it in registers, so the tile and the bulk store hold OutT.
+template <int P, int NQ, int PHS, int NS, int WMAX, int MINB, typename OutT>
 __global__ void __launch_bounds__((NQ *P *PHS + 31) / 32 * 32 + 64, MINB)
     roi_align_pipe_kernel(RoiLevels lv, int C, const float *__restrict__ rois, int K, int sr, int aligned, int mode, float finest,
-                          float *__restrict__ out, const float *__restrict__ bias, int bulk_store_flag,
+                          OutT *__restrict__ out, const float *__restrict__ bias, int bulk_store_flag,
                           const __grid_constant__ RoiTmaps tm, int cg32, const int *__restrict__ list,
                           const int *__restrict__ list_count) {
     constexpr int CC = NQ * 4;
@@ -508,8 +510,9 @@ __global__ void __launch_bounds__((NQ *P *PHS + 31) / 32 * 32 + 64, MINB)
     static_assert(P <= 16, "x bins on lanes 0..15, y bins on lanes 16..31 of the tap warp");
     extern __shared__ __align__(128) float smem[];
     float *s_ring = smem;                                   // [NS][WMAX][CC]
-    float *s_tile = s_ring + (size_t)NS * STAGE_FLOATS;     // [CC][S]
-    PipeSlot<P> *s_slot = reinterpret_cast<PipeSlot<P> *>(s_tile + CC * S); // [kPipeSlots]
+    float *s_tile_raw = s_ring + (size_t)NS * STAGE_FLOATS; // [CC][S] OutT (sized for fp32)
+    OutT *s_tile = reinterpret_cast<OutT *>(s_tile_raw);
+    PipeSlot<P> *s_slot = reinterpret_cast<PipeSlot<P> *>(s_tile_raw + CC * S); // [kPipeSlots]
     uint64_t *s_bar = reinterpret_cast<uint64_t *>(s_slot + kPipeSlots);    // full[NS], empty[NS], tfull[slots], tempty[slots]
     const uint32_t full0 = smem_u32(s_bar), empty0 = full0 + 8 * NS, tfull0 = empty0 + 8 * NS, tempty0 = tfull0 + 8 * kPipeSlots;
 
@@ -688,19 +691,19 @@ __global__ void __launch_bounds__((NQ *P *PHS + 31) / 32 * 32 + 64, MINB)
                 const float a0 = acc[i][0][0].x + bz.x, a1 = acc[i][0][0].y + bz.y, a2 = acc[i][0][1].x + bz.z, a3 = acc[i][0][1].y + bz.w;
                 // rotate (a0..a3) left by rot with two conditional stages (the predicates are per-thread constants)
                 const float b0 = rot2 ? a2 : a0, b1 = rot2 ? a3 : a1, b2 = rot2 ? a0 : a2, b3 = rot2 ? a1 : a3;
-                s_tile[toff[0] + i * P] = rot1 ? b1 : b0;
-                s_tile[toff[1] + i * P] = rot1 ? b2 : b1;
-                s_tile[toff[2] + i * P] = rot1 ? b3 : b2;
-                s_tile[toff[3] + i * P] = rot1 ? b0 : b3;
+                s_tile[toff[0] + i * P] = to_out<OutT>(rot1 ? b1 : b0);
+                s_tile[toff[1] + i * P] = to_out<OutT>(rot1 ? b2 : b1);
+                s_tile[toff[2] + i * P] = to_out<OutT>(rot1 ? b3 : b2);
+                s_tile[toff[3] + i * P] = to_out<OutT>(rot1 ? b0 : b3);
                 acc[i][0][0] = acc[i][0][1] = make_float2(0.f, 0.f);
             }
         }
-        float *outp = out + ((size_t)k * C + c0) * PP;
+        OutT *outp = out + ((size_t)k * C + c0) * PP;
         if (kBulkStore) {
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // my tile writes become visible to the TMA engine
             asm volatile("bar.sync 1, %0;" ::"n"(NCONS) : "memory");
             if (tid == 0) {
-                tma_bulk_s2g(outp, smem_u32(s_tile), CC * PP * 4);
+                tma_bulk_s2g(outp, smem_u32(s_tile), CC * PP * sizeof(OutT));   // 16-bit: CC >= 32, still a multiple of 16 B
                 tma_store_wait_read(); // only this thread waits; the others are already on the next unit's rows
             }
         } else {
@@ -709,12 +712,12 @@ __global__ void __launch_bounds__((NQ *P *PHS + 31) / 32 * 32 + 64, MINB)
             if (bulk_store_flag & 2) { // A/B: conflict-free scalar reads of the padded tile, 32-bit coalesced stores
                 for (int e = tid; e < CC * PP; e += NCONS) {
                     const int c = e / PP;
-                    __stcs(outp + e, s_tile[c * S + (e - c * PP)]);
+                    st_stream1(outp + e, s_tile[c * S + (e - c * PP)]);
                 }
             } else
             for (int i = tid; i < N4; i += NCONS) {
                 int c = (4 * i) / PP, e = 4 * i - c * PP;
-                float t[4];
+                OutT t[4];
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     t[u] = s_tile[c * S + e];
@@ -723,7 +726,7 @@ __global__ void __launch_bounds__((NQ *P *PHS + 31) / 32 * 32 + 64, MINB)
                         ++c;
                     }
                 }
-                st_stream_f4(outp + 4 * i, make_float4(t[0], t[1], t[2], t[3]));
+                st_stream4(outp + 4 * i, t[0], t[1], t[2], t[3]);
             }
         }
     };
@@ -858,9 +861,9 @@ static bool build_tmaps(const RoiLevels &lv, int B, int C, int CC, RoiTmaps *tm)
     return true;
 }
 
-template <int P, int NQ, int PHS, int NS, int WMAX, int MINB>
+template <int P, int NQ, int PHS, int NS, int WMAX, int MINB, typename OutT>
 static int launch_pipe(const RoiLevels &lv, int B, int C, const float *rois, int K, int sr, int aligned, int mode, float finest,
-                       float *out, const float *bias, cudaStream_t st, int cg32 = 0, const int *list = nullptr,
+                       OutT *out, const float *bias, cudaStream_t st, int cg32 = 0, const int *list = nullptr,
                        const int *list_count = nullptr) {
     static int grid_cache[kNuhtcMaxDevices] = {0};
     int &grid_cached = grid_cache[nuhtc_device()];
@@ -874,7 +877,7 @@ static int launch_pipe(const RoiLevels &lv, int B, int C, const float *rois, int
     const size_t smem = sizeof(float) * ((size_t)NS * WMAX * NQ * 4 + NQ * 4 * ((P == 14 && NQ == 32) ? P * P : SepCfg<P>::S)) +
                         kPipeSlots * sizeof(PipeSlot<P>) +
                         sizeof(uint64_t) * (2 * NS + 2 * kPipeSlots) + 128;
-    auto kern = roi_align_pipe_kernel<P, NQ, PHS, NS, WMAX, MINB>;
+    auto kern = roi_align_pipe_kernel<P, NQ, PHS, NS, WMAX, MINB, OutT>;
     constexpr int nthreads = (NQ * P * PHS + 31) / 32 * 32 + 64;
     if (!grid_cached) {
         NUHTC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1000,8 +1003,9 @@ NUHTC_API int nuhtc_roi_align_fwd(const float *const *feats, const int *H, const
 
 
 // per-RoI kernel on the channel-group layout: every RoI (list == nullptr) or the RoIs of a device-side list
+template <typename OutT>
 static int launch_sep_cg32(const RoiLevels &lv, int B, int C, const float *rois, int K, int P, int sr, int aligned, int mode,
-                           float finest, float *out, const float *bias, cudaStream_t st, const int *list,
+                           float finest, OutT *out, const float *bias, cudaStream_t st, const int *list,
                            const int *list_count) {
     // Pipelined kernel first: the window rows arrive through bulk copies (one per channel group and row), so a RoI's
     // latency is one ring fill instead of a chain of dependent global loads per row.  NUHTC_RA_PIPE=0: A/B switch.
@@ -1034,19 +1038,47 @@ NUHTC_API size_t nuhtc_roi_align_workspace_bytes(const int *H, const int *W, int
     return roi_strip_workspace_bytes(H, W, L, B, K, PH);
 }
 
-NUHTC_API int nuhtc_to_cg32(const float *in, float *out, int B, int C, int H, int W, int channels_last, void *stream) {
-    NUHTC_CHECK_ARG(B >= 0 && C >= 32 && C % 32 == 0 && H >= 1 && W >= 1, "to_cg32: bad sizes (C must be a multiple of 32)");
-    if (B == 0) return NUHTC_OK;
-    NUHTC_CHECK_ARG(in && out && ((uintptr_t)in % 16 == 0) && ((uintptr_t)out % 16 == 0), "to_cg32: null or misaligned pointer");
-    NUHTC_CHECK_ARG(channels_last || (H * W) % 4 == 0, "to_cg32: H*W must be a multiple of 4 for an NCHW source");
-    NUHTC_CHECK_ARG(C / 32 <= 65535 && B <= 65535, "to_cg32: C or B too large");
-    return roi_to_cg32(in, out, B, C, H, W, channels_last, (cudaStream_t)stream);
+static size_t dtype_size(int dtype) {   // 0: not a NUHTC_DTYPE_* code
+    return dtype == NUHTC_DTYPE_F32 ? 4 : (dtype == NUHTC_DTYPE_F16 || dtype == NUHTC_DTYPE_BF16) ? 2 : 0;
 }
 
-NUHTC_API int nuhtc_roi_align_cg32(const float *const *feats, const int *H, const int *W, const float *scale, int L, int B,
-                                   int C, const float *rois, int K, int PH, int PW, int sampling_ratio, int aligned, int mode,
-                                   float finest_scale, const int *pool2, float *out, const float *bias, void *ws, size_t ws_bytes,
-                                   void *stream) {
+NUHTC_API int nuhtc_to_cg32_dt(const void *in, int in_dtype, float *out, int B, int C, int H, int W, int channels_last, void *stream) {
+    const size_t es = dtype_size(in_dtype);
+    NUHTC_CHECK_ARG(es != 0, "to_cg32: unknown dtype code %d", in_dtype);
+    NUHTC_CHECK_ARG(B >= 0 && C >= 32 && C % 32 == 0 && H >= 1 && W >= 1, "to_cg32: bad sizes (C must be a multiple of 32)");
+    if (B == 0) return NUHTC_OK;
+    // the staging kernels read four input elements at a time and write 16-byte vectors
+    NUHTC_CHECK_ARG(in && out && ((uintptr_t)in % (4 * es) == 0) && ((uintptr_t)out % 16 == 0), "to_cg32: null or misaligned pointer");
+    NUHTC_CHECK_ARG(channels_last || (H * W) % 4 == 0, "to_cg32: H*W must be a multiple of 4 for an NCHW source");
+    NUHTC_CHECK_ARG(C / 32 <= 65535 && B <= 65535, "to_cg32: C or B too large");
+    return roi_to_cg32(in, in_dtype, out, B, C, H, W, channels_last, (cudaStream_t)stream);
+}
+
+NUHTC_API int nuhtc_to_cg32(const float *in, float *out, int B, int C, int H, int W, int channels_last, void *stream) {
+    return nuhtc_to_cg32_dt(in, NUHTC_DTYPE_F32, out, B, C, H, W, channels_last, stream);
+}
+
+template <typename OutT>
+static int roi_align_cg32_run(const RoiLevels &lv, int B, int C, const float *rois, int K, int PH, int PW, int sampling_ratio,
+                              int aligned, int mode, float finest_scale, OutT *out, int out_dtype, const float *bias, void *ws,
+                              size_t ws_bytes, cudaStream_t st) {
+    static const bool no_strip = getenv("NUHTC_RA_STRIP") && getenv("NUHTC_RA_STRIP")[0] == '0';   // A/B: per-RoI kernel only
+    if (roi_strip_supported(C, PH, PW, mode, lv.L) && !no_strip) {
+        const int *left = nullptr, *left_count = nullptr;
+        const int rc = roi_strip_forward(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, out_dtype, bias, ws,
+                                         ws_bytes, st, &left, &left_count);
+        if (rc == NUHTC_OK)
+            return launch_sep_cg32(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, bias, st, left, left_count);
+        if (rc != 1) return rc;   // 1: the levels are too large for the strip binning -> every RoI through the per-RoI kernel
+    }
+    return launch_sep_cg32(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, bias, st, nullptr, nullptr);
+}
+
+NUHTC_API int nuhtc_roi_align_cg32_dt(const float *const *feats, const int *H, const int *W, const float *scale, int L, int B,
+                                      int C, const float *rois, int K, int PH, int PW, int sampling_ratio, int aligned, int mode,
+                                      float finest_scale, const int *pool2, void *out, int out_dtype, const float *bias, void *ws,
+                                      size_t ws_bytes, void *stream) {
+    NUHTC_CHECK_ARG(dtype_size(out_dtype) != 0, "roi_align_cg32: unknown dtype code %d", out_dtype);
     NUHTC_CHECK_ARG(L >= 1 && L <= NUHTC_MAX_LEVELS, "roi_align_cg32: L=%d out of range", L);
     NUHTC_CHECK_ARG(PH == PW && (PH == 7 || PH == 14) && C >= 32 && C % 32 == 0 && B >= 0 && K >= 0,
                     "roi_align_cg32: needs PH == PW in {7, 14} and C %% 32 == 0 (PH=%d PW=%d C=%d)", PH, PW, C);
@@ -1067,16 +1099,25 @@ NUHTC_API int nuhtc_roi_align_cg32(const float *const *feats, const int *H, cons
     }
     NUHTC_CHECK_ARG((uintptr_t)out % 16 == 0, "roi_align_cg32: out must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
-    static const bool no_strip = getenv("NUHTC_RA_STRIP") && getenv("NUHTC_RA_STRIP")[0] == '0';   // A/B: per-RoI kernel only
-    if (roi_strip_supported(C, PH, PW, mode, L) && !no_strip) {
-        const int *left = nullptr, *left_count = nullptr;
-        const int rc = roi_strip_forward(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, bias, ws, ws_bytes,
-                                         st, &left, &left_count);
-        if (rc == NUHTC_OK)
-            return launch_sep_cg32(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, bias, st, left, left_count);
-        if (rc != 1) return rc;   // 1: the levels are too large for the strip binning -> every RoI through the per-RoI kernel
+    switch (out_dtype) {
+        case NUHTC_DTYPE_F16:
+            return roi_align_cg32_run(lv, B, C, rois, K, PH, PW, sampling_ratio, aligned, mode, finest_scale, static_cast<__half *>(out),
+                                      out_dtype, bias, ws, ws_bytes, st);
+        case NUHTC_DTYPE_BF16:
+            return roi_align_cg32_run(lv, B, C, rois, K, PH, PW, sampling_ratio, aligned, mode, finest_scale,
+                                      static_cast<__nv_bfloat16 *>(out), out_dtype, bias, ws, ws_bytes, st);
+        default:
+            return roi_align_cg32_run(lv, B, C, rois, K, PH, PW, sampling_ratio, aligned, mode, finest_scale, static_cast<float *>(out),
+                                      out_dtype, bias, ws, ws_bytes, st);
     }
-    return launch_sep_cg32(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, bias, st, nullptr, nullptr);
+}
+
+NUHTC_API int nuhtc_roi_align_cg32(const float *const *feats, const int *H, const int *W, const float *scale, int L, int B,
+                                   int C, const float *rois, int K, int PH, int PW, int sampling_ratio, int aligned, int mode,
+                                   float finest_scale, const int *pool2, float *out, const float *bias, void *ws, size_t ws_bytes,
+                                   void *stream) {
+    return nuhtc_roi_align_cg32_dt(feats, H, W, scale, L, B, C, rois, K, PH, PW, sampling_ratio, aligned, mode, finest_scale, pool2,
+                                   out, NUHTC_DTYPE_F32, bias, ws, ws_bytes, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

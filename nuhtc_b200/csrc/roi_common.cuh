@@ -2,6 +2,9 @@
 // reference's fp32 op order, per-axis tap tables, packed fp32x2 FMA, mbarrier / TMA bulk-copy wrappers.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 
 struct RoiLevels {
@@ -217,3 +220,45 @@ __device__ __forceinline__ void tma_bulk_s2g(void *dst, uint32_t src, uint32_t b
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
+
+// ---- element types (NUHTC_DTYPE_*) --------------------------------------------------------------------------------------
+// Half-precision levels are upcast exactly while they are staged; every RoIAlign kernel computes in fp32 and rounds each
+// output value once, round-to-nearest-even, to the output type at its final store (mmcv's force_fp32(out_fp16=True)).
+template <typename T> __device__ __forceinline__ T to_out(float v);
+template <> __device__ __forceinline__ float to_out<float>(float v) { return v; }
+template <> __device__ __forceinline__ __half to_out<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 to_out<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+
+__device__ __forceinline__ uint32_t bits16(__half v) { return __half_as_ushort(v); }
+__device__ __forceinline__ uint32_t bits16(__nv_bfloat16 v) { return __bfloat16_as_ushort(v); }
+
+// four consecutive output elements, streaming store: 16 bytes for fp32, 8 bytes for the 16-bit types
+__device__ __forceinline__ void st_stream4(float *p, float a, float b, float c, float d) { st_stream_f4(p, make_float4(a, b, c, d)); }
+template <typename T>
+__device__ __forceinline__ void st_stream4(T *p, T a, T b, T c, T d) {
+    asm volatile("st.global.cs.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(bits16(a) | bits16(b) << 16), "r"(bits16(c) | bits16(d) << 16)
+                 : "memory");
+}
+__device__ __forceinline__ void st_stream1(float *p, float v) { __stcs(p, v); }
+template <typename T>
+__device__ __forceinline__ void st_stream1(T *p, T v) {
+    asm volatile("st.global.cs.u16 [%0], %1;" ::"l"(p), "h"((unsigned short)bits16(v)) : "memory");
+}
+
+// four consecutive input elements, upcast exactly to fp32 (bf16: a 16-bit shift, so subnormals stay exact)
+__device__ __forceinline__ float4 ldg_in4(const float *p) { return ldg_f4(p); }
+__device__ __forceinline__ float4 ldg_in4(const __half *p) {
+    const uint2 u = __ldg(reinterpret_cast<const uint2 *>(p));
+    const float2 lo = __half22float2(*reinterpret_cast<const __half2 *>(&u.x)), hi = __half22float2(*reinterpret_cast<const __half2 *>(&u.y));
+    return make_float4(lo.x, lo.y, hi.x, hi.y);
+}
+__device__ __forceinline__ float4 ldg_in4(const __nv_bfloat16 *p) {
+    const uint2 u = __ldg(reinterpret_cast<const uint2 *>(p));
+    return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
+                       __uint_as_float(u.y & 0xffff0000u));
+}
+__device__ __forceinline__ float ldg_in1(const float *p) { return __ldg(p); }
+__device__ __forceinline__ float ldg_in1(const __half *p) { return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short *>(p)))); }
+__device__ __forceinline__ float ldg_in1(const __nv_bfloat16 *p) {
+    return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short *>(p)) << 16);
+}

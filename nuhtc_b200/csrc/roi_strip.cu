@@ -83,7 +83,7 @@ struct StripArgs {
     int nkeys, nbins;
     int dbg;           // measurement switches (NUHTC_RA_DBG): 1 skip the pooling arithmetic + stores, 2 skip the stores only
     const float *rois;
-    float *out;
+    void *out;         // [K][C][P][P] elements of the kernel's OutT
     const float *bias;
     // workspace
     int *item_key;     // [K] sort key of the item, -1: leftover
@@ -479,6 +479,7 @@ struct Strip7Cfg {
     static_assert(NR >= kRMax + 2, "the ring must hold the tallest window plus some slack");
 };
 
+template <typename OutT>
 __global__ void __launch_bounds__(Strip7Cfg::NTHREADS, 1) roi_align_strip7_kernel(const __grid_constant__ StripArgs a) {
     using Cfg = Strip7Cfg;
     using Rec = StripRec<7>;
@@ -519,7 +520,7 @@ __global__ void __launch_bounds__(Strip7Cfg::NTHREADS, 1) roi_align_strip7_kerne
     // this lane keeps its HIGH slice in register set 0; the four idle lanes share a quarter-warp with column 6 (even: low
     // half of its cell) and must read a high half, or that phase of every tap load is a 2-way bank conflict
     const bool odd = worker ? (pw & 1) != 0 : true;
-    float *tile = s_tile + cw * Cfg::TILE_FLOATS;
+    OutT *tile = reinterpret_cast<OutT *>(s_tile + cw * Cfg::TILE_FLOATS);   // a 16-bit tile fills half of its slot
     Rec *recs = s_rec + cw * 2;
     const uint32_t rf0 = B.rfull0 + 8 * (cw * 2);
     unsigned rec_uses[2] = {0u, 0u};
@@ -696,8 +697,9 @@ __global__ void __launch_bounds__(Strip7Cfg::NTHREADS, 1) roi_align_strip7_kerne
                 }
             }
             passed = max(passed, y0 + rel);
-            // ---- flush: two 16-channel slices through the warp's tile, one asynchronous bulk store each
-            float *outp = a.out + ((size_t)k * a.C + (size_t)cg * kCG) * PP;
+            // ---- flush: two 16-channel slices through the warp's tile, one asynchronous bulk store each (the values are
+            // rounded to OutT in registers: a 16-bit slice is 1568 B, still a multiple of the bulk copy's 16 bytes)
+            OutT *outp = static_cast<OutT *>(a.out) + ((size_t)k * a.C + (size_t)cg * kCG) * PP;
             auto flush = [&](auto HASBIAS) {
                 constexpr bool kBias = decltype(HASBIAS)::value;
 #pragma unroll
@@ -708,7 +710,7 @@ __global__ void __launch_bounds__(Strip7Cfg::NTHREADS, 1) roi_align_strip7_kerne
                         const bool hi = odd != (f == 1);   // slice f sits in register set f ^ odd
                         float4 bz = make_float4(0.f, 0.f, 0.f, 0.f);
                         if (kBias) bz = ldg_f4(a.bias + (size_t)k * a.C + cg * kCG + 16 * f + 4 * q);
-                        float *tp = tile + (4 * q) * PP + pw;
+                        OutT *tp = tile + (4 * q) * PP + pw;
 #pragma unroll
                         for (int i = 0; i < P; ++i) {
                             float a0 = hi ? acc[1][i][0].x : acc[0][i][0].x, a1 = hi ? acc[1][i][0].y : acc[0][i][0].y;
@@ -716,16 +718,16 @@ __global__ void __launch_bounds__(Strip7Cfg::NTHREADS, 1) roi_align_strip7_kerne
                             if (kBias) {
                                 a0 += bz.x; a1 += bz.y; a2 += bz.z; a3 += bz.w;
                             }
-                            tp[i * P] = a0;
-                            tp[i * P + PP] = a1;
-                            tp[i * P + 2 * PP] = a2;
-                            tp[i * P + 3 * PP] = a3;
+                            tp[i * P] = to_out<OutT>(a0);
+                            tp[i * P + PP] = to_out<OutT>(a1);
+                            tp[i * P + 2 * PP] = to_out<OutT>(a2);
+                            tp[i * P + 3 * PP] = to_out<OutT>(a3);
                         }
                     }
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                     __syncwarp();
                     if (lane == 0) {
-                        tma_bulk_s2g(outp + (size_t)f * Cfg::TILE_FLOATS, smem_u32(tile), Cfg::TILE_FLOATS * 4);
+                        tma_bulk_s2g(outp + (size_t)f * Cfg::TILE_FLOATS, smem_u32(tile), Cfg::TILE_FLOATS * sizeof(OutT));
                         store_pending = true;
                     }
                 }
@@ -763,6 +765,7 @@ struct Strip14Cfg {
     static_assert(NR >= kRMax + 2, "the ring must hold the tallest window plus some slack");
 };
 
+template <typename OutT>
 __global__ void __launch_bounds__(Strip14Cfg::NTHREADS, 1) roi_align_strip14_kernel(const __grid_constant__ StripArgs a) {
     using Cfg = Strip14Cfg;
     using Rec = StripRec<14>;
@@ -802,7 +805,7 @@ __global__ void __launch_bounds__(Strip14Cfg::NTHREADS, 1) roi_align_strip14_ker
     const int team = ct / TEAM, tt = ct % TEAM, twarp = tt >> 5, lane = tt & 31;
     const bool worker = tt < 8 * P;
     const int q = tt & 7, pw = worker ? tt >> 3 : 0;
-    float *tile = s_tile + team * Cfg::TILE_FLOATS;
+    OutT *tile = reinterpret_cast<OutT *>(s_tile + team * Cfg::TILE_FLOATS);   // a 16-bit tile fills half of its slot
     Rec *recs = s_rec + team * 2;
     const uint32_t rf0 = B.rfull0 + 8 * (team * 2);
     const int bar_id = 1 + team;
@@ -949,7 +952,7 @@ __global__ void __launch_bounds__(Strip14Cfg::NTHREADS, 1) roi_align_strip14_ker
             // swapped order (a rotation by two = a renaming of acc[.][0] / acc[.][1], one select per value), which leaves quad q
             // and q + 4 on the same bank -- a 2-way conflict, i.e. as many wavefronts as two half-warp passes would take at
             // half the issue slots (every warp holds quads of both halves, so a split pass is issued twice by every warp).
-            float *outp = a.out + ((size_t)k * a.C + (size_t)cg * kCG) * PP;
+            OutT *outp = static_cast<OutT *>(a.out) + ((size_t)k * a.C + (size_t)cg * kCG) * PP;
             auto flush = [&](auto HASBIAS) {
                 constexpr bool kBias = decltype(HASBIAS)::value;
                 if (tt == 0 && store_pending) tma_store_wait_read();
@@ -958,8 +961,8 @@ __global__ void __launch_bounds__(Strip14Cfg::NTHREADS, 1) roi_align_strip14_ker
                     const int cl = 4 * q;
                     float4 bz = make_float4(0.f, 0.f, 0.f, 0.f);
                     if (kBias) bz = ldg_f4(a.bias + (size_t)k * a.C + cg * kCG + 4 * q);
-                    float *tp = tile + pw;
-                    float *tlo = tp + (cl + (r2 ? 2 : 0)) * PP, *thi = tp + (cl + (r2 ? 0 : 2)) * PP;
+                    OutT *tp = tile + pw;
+                    OutT *tlo = tp + (cl + (r2 ? 2 : 0)) * PP, *thi = tp + (cl + (r2 ? 0 : 2)) * PP;
 #pragma unroll
                     for (int i = 0; i < P; ++i) {
                         float a0 = acc[i][0].x, a1 = acc[i][0].y, a2 = acc[i][1].x, a3 = acc[i][1].y;
@@ -967,16 +970,16 @@ __global__ void __launch_bounds__(Strip14Cfg::NTHREADS, 1) roi_align_strip14_ker
                             a0 += bz.x; a1 += bz.y; a2 += bz.z; a3 += bz.w;
                         }
                         // first instruction pair: channels cl+0,1 for quads 0,1 (mod 4), cl+2,3 for quads 2,3
-                        tlo[i * P] = r2 ? a2 : a0;
-                        tlo[i * P + PP] = r2 ? a3 : a1;
-                        thi[i * P] = r2 ? a0 : a2;
-                        thi[i * P + PP] = r2 ? a1 : a3;
+                        tlo[i * P] = to_out<OutT>(r2 ? a2 : a0);
+                        tlo[i * P + PP] = to_out<OutT>(r2 ? a3 : a1);
+                        thi[i * P] = to_out<OutT>(r2 ? a0 : a2);
+                        thi[i * P + PP] = to_out<OutT>(r2 ? a1 : a3);
                     }
                 }
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 team_sync();
                 if (tt == 0) {
-                    tma_bulk_s2g(outp, smem_u32(tile), Cfg::TILE_FLOATS * 4);
+                    tma_bulk_s2g(outp, smem_u32(tile), Cfg::TILE_FLOATS * sizeof(OutT));
                     store_pending = true;
                 }
             };
@@ -1005,22 +1008,24 @@ static size_t strip14_smem_bytes() {
 // ---------------------------------------------------------------------------------------------
 // layout staging: NCHW / channels_last -> [B][C/32][H][W][32]
 // ---------------------------------------------------------------------------------------------
-// 32 channels x 64 pixels per CTA: reads 64 contiguous floats per channel, writes one contiguous 8 KB chunk
-__global__ void __launch_bounds__(256) nchw_to_cg32_kernel(const float *__restrict__ in, float *__restrict__ out, int C, int HW) {
+// 32 channels x 64 pixels per CTA: reads 64 contiguous elements per channel, writes one contiguous 8 KB chunk.  InT: fp32,
+// or fp16 / bf16 upcast exactly on the way in (the staged buffer is fp32 whatever the source type)
+template <typename InT>
+__global__ void __launch_bounds__(256) nchw_to_cg32_kernel(const InT *__restrict__ in, float *__restrict__ out, int C, int HW) {
     __shared__ float tile[32][65];
     const int b = blockIdx.z, cg = blockIdx.y, hw0 = blockIdx.x * 64;
     const int t = threadIdx.x;
-    const float *src = in + ((size_t)b * C + cg * 32) * HW;
-    {   // thread = (channel r + 16k, pixel quad q): 128-bit loads
+    const InT *src = in + ((size_t)b * C + cg * 32) * HW;
+    {   // thread = (channel r + 16k, pixel quad q): 128-bit loads (64-bit for 16-bit sources)
         const int r = t >> 4, q = (t & 15) * 4;
 #pragma unroll
         for (int k = 0; k < 2; ++k) {
             const int c = r + 16 * k, hw = hw0 + q;
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (hw + 3 < HW) v = ldg_f4(src + (size_t)c * HW + hw);
+            if (hw + 3 < HW) v = ldg_in4(src + (size_t)c * HW + hw);
             else
                 for (int e = 0; e < 4; ++e)
-                    if (hw + e < HW) (&v.x)[e] = __ldg(src + (size_t)c * HW + hw + e);
+                    if (hw + e < HW) (&v.x)[e] = ldg_in1(src + (size_t)c * HW + hw + e);
             tile[c][q] = v.x; tile[c][q + 1] = v.y; tile[c][q + 2] = v.z; tile[c][q + 3] = v.w;
         }
     }
@@ -1038,7 +1043,8 @@ __global__ void __launch_bounds__(256) nchw_to_cg32_kernel(const float *__restri
 }
 
 // channels_last source: [B][HW][C] -> [B][C/32][HW][32], a pure 128-byte-line permutation
-__global__ void __launch_bounds__(256) nhwc_to_cg32_kernel(const float *__restrict__ in, float *__restrict__ out, int C, long HW, long total4) {
+template <typename InT>
+__global__ void __launch_bounds__(256) nhwc_to_cg32_kernel(const InT *__restrict__ in, float *__restrict__ out, int C, long HW, long total4) {
     for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < total4; i += (long)gridDim.x * blockDim.x) {
         // i indexes float4s of the OUTPUT: ((b*CG + cg)*HW + hw)*8 + q
         const int q = (int)(i & 7);
@@ -1047,7 +1053,7 @@ __global__ void __launch_bounds__(256) nhwc_to_cg32_kernel(const float *__restri
         const long bc = r / HW;
         const int cg = (int)(bc % (C / 32));
         const long b = bc / (C / 32);
-        const float4 v = ldg_f4(in + ((size_t)(b * HW + hw)) * C + cg * 32 + q * 4);
+        const float4 v = ldg_in4(in + ((size_t)(b * HW + hw)) * C + cg * 32 + q * 4);
         *reinterpret_cast<float4 *>(out + (size_t)i * 4) = v;
     }
 }
@@ -1119,14 +1125,14 @@ bool roi_strip_supported(int C, int PH, int PW, int mode, int L) {
     return PH == PW && (PH == 7 || PH == 14) && C % 32 == 0 && C >= 32 && (mode == NUHTC_ROI_ROUTE || L == 1);
 }
 
-template <int P>
+template <int P, typename OutT>
 static int strip_launch(StripArgs &a, const RoiLevels &lv, cudaStream_t st, const StripWs &w, char *ws) {
     static bool attr_done[kNuhtcMaxDevices] = {false};
     const int dev = nuhtc_device();
     const size_t smem = P == 7 ? strip7_smem_bytes() : strip14_smem_bytes();
     if (!attr_done[dev]) {
-        if (P == 7) NUHTC_CUDA(cudaFuncSetAttribute(roi_align_strip7_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        else NUHTC_CUDA(cudaFuncSetAttribute(roi_align_strip14_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (P == 7) NUHTC_CUDA(cudaFuncSetAttribute(roi_align_strip7_kernel<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        else NUHTC_CUDA(cudaFuncSetAttribute(roi_align_strip14_kernel<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_done[dev] = true;
     }
     NUHTC_CUDA(cudaMemsetAsync(ws + w.counters, 0, w.cursor - w.counters, st));
@@ -1143,8 +1149,8 @@ static int strip_launch(StripArgs &a, const RoiLevels &lv, cudaStream_t st, cons
     NUHTC_LAUNCH_CHECK();
     strip_records_kernel<P><<<gblocks, 256, 0, st>>>(a);
     NUHTC_LAUNCH_CHECK();
-    if (P == 7) roi_align_strip7_kernel<<<nuhtc_sm_count(), Strip7Cfg::NTHREADS, smem, st>>>(a);
-    else roi_align_strip14_kernel<<<nuhtc_sm_count(), Strip14Cfg::NTHREADS, smem, st>>>(a);
+    if (P == 7) roi_align_strip7_kernel<OutT><<<nuhtc_sm_count(), Strip7Cfg::NTHREADS, smem, st>>>(a);
+    else roi_align_strip14_kernel<OutT><<<nuhtc_sm_count(), Strip14Cfg::NTHREADS, smem, st>>>(a);
     NUHTC_LAUNCH_CHECK();
     (void)lv;
     return NUHTC_OK;
@@ -1153,7 +1159,7 @@ static int strip_launch(StripArgs &a, const RoiLevels &lv, cudaStream_t st, cons
 // Fills `a` and runs prepass + strip kernel; the caller then runs its per-RoI kernel over the leftover list
 // (*leftover, *leftover_count are device pointers into the workspace).
 int roi_strip_forward(const RoiLevels &lv, int B, int C, const float *rois, int K, int P, int sr, int aligned, int mode,
-                      float finest, float *out, const float *bias, void *ws_, size_t ws_bytes, cudaStream_t st,
+                      float finest, void *out, int out_dtype, const float *bias, void *ws_, size_t ws_bytes, cudaStream_t st,
                       const int **leftover, const int **leftover_count) {
     StripArgs a;
     memset(&a, 0, sizeof a);
@@ -1197,21 +1203,35 @@ int roi_strip_forward(const RoiLevels &lv, int B, int C, const float *rois, int 
     a.records = ws + w.records;
     *leftover = a.leftover;
     *leftover_count = a.counters + 2;
-    return P == 7 ? strip_launch<7>(a, lv, st, w, ws) : strip_launch<14>(a, lv, st, w, ws);
+    switch (out_dtype) {
+        case NUHTC_DTYPE_F16: return P == 7 ? strip_launch<7, __half>(a, lv, st, w, ws) : strip_launch<14, __half>(a, lv, st, w, ws);
+        case NUHTC_DTYPE_BF16:
+            return P == 7 ? strip_launch<7, __nv_bfloat16>(a, lv, st, w, ws) : strip_launch<14, __nv_bfloat16>(a, lv, st, w, ws);
+        default: return P == 7 ? strip_launch<7, float>(a, lv, st, w, ws) : strip_launch<14, float>(a, lv, st, w, ws);
+    }
 }
 
-int roi_to_cg32(const float *in, float *out, int B, int C, int H, int W, int channels_last, cudaStream_t st) {
+template <typename InT>
+static int to_cg32_launch(const InT *in, float *out, int B, int C, int H, int W, int channels_last, cudaStream_t st) {
     const int HW = H * W;
     if (channels_last) {
         const long total4 = (long)B * C * HW / 4;
         long blocks = (total4 + 255) / 256;
         const long cap = (long)nuhtc_sm_count() * 16;
         if (blocks > cap) blocks = cap;
-        nhwc_to_cg32_kernel<<<(unsigned)blocks, 256, 0, st>>>(in, out, C, HW, total4);
+        nhwc_to_cg32_kernel<InT><<<(unsigned)blocks, 256, 0, st>>>(in, out, C, HW, total4);
     } else {
         dim3 grid((HW + 63) / 64, C / 32, B);
-        nchw_to_cg32_kernel<<<grid, 256, 0, st>>>(in, out, C, HW);
+        nchw_to_cg32_kernel<InT><<<grid, 256, 0, st>>>(in, out, C, HW);
     }
     NUHTC_LAUNCH_CHECK();
     return NUHTC_OK;
+}
+
+int roi_to_cg32(const void *in, int in_dtype, float *out, int B, int C, int H, int W, int channels_last, cudaStream_t st) {
+    switch (in_dtype) {
+        case NUHTC_DTYPE_F16: return to_cg32_launch(static_cast<const __half *>(in), out, B, C, H, W, channels_last, st);
+        case NUHTC_DTYPE_BF16: return to_cg32_launch(static_cast<const __nv_bfloat16 *>(in), out, B, C, H, W, channels_last, st);
+        default: return to_cg32_launch(static_cast<const float *>(in), out, B, C, H, W, channels_last, st);
+    }
 }

@@ -20,6 +20,9 @@ Head protocol (what the wrapper needs from the caller's modules -- mmdet's heads
         (default softmax; ``seesaw_activation`` is the NuHTC configs' SeesawLoss.get_activation)
   mask_head(mask_feats [D,C,14,14]) -> logits [D,1,h,w]   (class-agnostic, as every NuHTC config sets)
   semantic_head(x) -> (semantic_pred, semantic_feat)       (optional)
+
+Half precision: ``x`` and the semantic feature map may be fp16 or bf16 (mmcv's wrap_fp16_model, torch.autocast); the
+heads then receive RoI features in that dtype and the result format is unchanged (fp32 boxes, bool masks).
 """
 from __future__ import annotations
 
@@ -82,6 +85,9 @@ class HybridTaskCascadeRoIHead_Lite:
             from .watershed import watershed_proposal as _ws
 
             def watershed_proposal(semantic_pred, proposal_list, img_shape):
+                if semantic_pred.dtype != torch.float32:
+                    raise NotImplementedError("watershed_proposal=True needs an fp32 semantic prediction: its blur and threshold "
+                                              f"would otherwise run in {semantic_pred.dtype}, not as the fp32 reference does")
                 return _ws(semantic_pred, proposal_list=proposal_list, img_shape=img_shape, min_area=10, thres=0)[0]
         self.watershed_proposal = watershed_proposal or None
         self.test_cfg = dict(test_cfg)

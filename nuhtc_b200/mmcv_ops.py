@@ -72,7 +72,7 @@ class layout_cache:
 
 def _cached(x: torch.Tensor, kind: str, make):
     use = _LAYOUT_CACHE_ON[0] and not torch.cuda.is_current_stream_capturing()
-    key = (kind, x.data_ptr(), x._version, tuple(x.shape), tuple(x.stride()), x.device.index)
+    key = (kind, x.data_ptr(), x._version, tuple(x.shape), tuple(x.stride()), x.dtype, x.device.index)
     if use and key in _LAYOUT_CACHE:
         _LAYOUT_CACHE.move_to_end(key)
         return _LAYOUT_CACHE[key][1]
@@ -103,10 +103,23 @@ def to_nhwc(x: torch.Tensor) -> torch.Tensor:
     return _cached(x, "nhwc", make)
 
 
+def _levels_dtype(levels: Sequence[torch.Tensor]) -> torch.dtype:
+    """The one element type of a set of feature maps: fp32, fp16 or bf16 (ValueError otherwise)."""
+    dts = {f.dtype for f in levels}
+    if len(dts) != 1:
+        raise ValueError(f"feature levels must share one dtype, got {sorted(str(d) for d in dts)}")
+    dt = dts.pop()
+    if dt not in L.DTYPE_CODES:
+        raise ValueError(f"feature levels must be float32, float16 or bfloat16, got {dt}")
+    return dt
+
+
 def to_cg32(x: torch.Tensor) -> torch.Tensor:
-    """[B,C,H,W] fp32 CUDA, C % 32 == 0 (NCHW-contiguous or channels_last) -> [B, C/32, H, W, 32] buffer."""
+    """[B,C,H,W] fp32, fp16 or bf16 CUDA, C % 32 == 0 (NCHW-contiguous or channels_last) -> [B, C/32, H, W, 32] fp32
+    buffer.  A half-precision map is upcast exactly while it is staged: the buffer equals ``to_cg32(x.float())``."""
     L.require_cuda(x, "input")
-    assert x.dim() == 4 and x.dtype == torch.float32, "expected a 4-D fp32 feature map"
+    assert x.dim() == 4, "expected a 4-D feature map"
+    code = L.DTYPE_CODES[_levels_dtype([x])]
     B, C, H, W = x.shape
     assert C % 32 == 0
     cl = x.permute(0, 2, 3, 1).is_contiguous() and not x.is_contiguous()
@@ -118,7 +131,8 @@ def to_cg32(x: torch.Tensor) -> torch.Tensor:
         out = torch.empty((B, C // 32, H, W, 32), dtype=torch.float32, device=x.device)
         if B > 0:
             with torch.cuda.device(x.device):
-                L.check(L.lib().nuhtc_to_cg32(x.data_ptr(), out.data_ptr(), B, C, H, W, int(cl), L.stream_ptr(x.device)), "to_cg32")
+                L.check(L.lib().nuhtc_to_cg32_dt(x.data_ptr(), code, out.data_ptr(), B, C, H, W, int(cl), L.stream_ptr(x.device)),
+                        "to_cg32")
             L.count("to_cg32")
         return out
     return _cached(x, "cg32", make)
@@ -130,7 +144,9 @@ def _fast_path_ok(C: int, ph: int, pw: int) -> bool:
 
 class StagedLevels:
     """FPN levels of one batch, laid out for the RoIAlign kernels.  Build it once per batch with ``stage_levels`` and pass
-    it wherever ``feats`` is accepted: the three cascade stages and the mask branch then share one re-layout."""
+    it wherever ``feats`` is accepted: the three cascade stages and the mask branch then share one re-layout.
+    The levels are fp32, fp16 or bf16, all of one dtype (``self.dtype``, the dtype of the RoI features pooled from them);
+    the staged CG32 buffers are fp32 either way."""
 
     def __init__(self, feats: Sequence[torch.Tensor]):
         f0 = feats[0]
@@ -139,7 +155,8 @@ class StagedLevels:
         self.device = f0.device
         for f in feats:
             L.require_cuda(f, "feats")
-            assert f.dtype == torch.float32 and f.shape[0] == self.B and f.shape[1] == self.C
+            assert f.shape[0] == self.B and f.shape[1] == self.C
+        self.dtype = _levels_dtype(feats)
         self.nchw = list(feats)
         self.cg32 = [to_cg32(f) for f in feats] if self.C % 32 == 0 else None
 
@@ -149,8 +166,10 @@ class StagedLevels:
     def cat(self, other: "StagedLevels") -> "StagedLevels":
         """these levels followed by `other`'s (same batch and channel count), e.g. FPN levels + the semantic feature map"""
         assert other.B == self.B and other.C == self.C
+        if other.dtype != self.dtype:
+            raise ValueError(f"feature levels must share one dtype, got {self.dtype} and {other.dtype}")
         o = object.__new__(StagedLevels)
-        o.B, o.C, o.device = self.B, self.C, self.device
+        o.B, o.C, o.device, o.dtype = self.B, self.C, self.device, self.dtype
         o.shapes = self.shapes + other.shapes
         o.nchw = self.nchw + other.nchw
         o.cg32 = None if (self.cg32 is None or other.cg32 is None) else self.cg32 + other.cg32
@@ -158,7 +177,7 @@ class StagedLevels:
 
     def sub(self, idx: Sequence[int]) -> "StagedLevels":
         o = object.__new__(StagedLevels)
-        o.B, o.C, o.device = self.B, self.C, self.device
+        o.B, o.C, o.device, o.dtype = self.B, self.C, self.device, self.dtype
         o.shapes = [self.shapes[i] for i in idx]
         o.nchw = [self.nchw[i] for i in idx]
         o.cg32 = None if self.cg32 is None else [self.cg32[i] for i in idx]
@@ -179,7 +198,12 @@ def roi_align_levels(feats, rois: torch.Tensor, output_size, spatial_scales: Seq
                   (single_level_roi_extractor.py:36-55); one level = plain roi_align.
     mode 'sum'  : every RoI is pooled on every level, results summed in level order
                   (AttentionRoIExtractor's RoIAlign branch, roi_extractors_cus.py:213-218,246).
-    feats: NCHW fp32 CUDA tensors [B,C,H_l,W_l] (NCHW-contiguous or channels_last), or a ``StagedLevels``.
+    feats: NCHW CUDA tensors [B,C,H_l,W_l] (NCHW-contiguous or channels_last), or a ``StagedLevels``; fp32, fp16 or bf16,
+           all levels of one dtype (ValueError otherwise).  The result has that dtype (a given ``out`` must have it too);
+           ``bias`` stays fp32.  Everything is computed in fp32 and each output value is rounded once to the levels'
+           dtype (mmcv's ``force_fp32(out_fp16=True)``).  On the channel-group path (impl 'auto', C % 32 == 0, 7x7 or
+           14x14) half levels are staged and stored natively; every other shape and impl runs the fp32 kernels between
+           ONE ``.float()`` of the levels and ONE rounding of the result (its copy into ``out``), both below.
     pool2: per level (mode 'sum'): the level enters as adaptive_avg_pool2d(RoIAlign(2P x 2P, sampling_ratio=0), P) -- the
            semantic branch of NuHTC's _bbox_forward -- pooled directly at P x P inside the same launch.
     impl : 'auto' (strip-shared kernels on the CG32 layout when the shape allows, else the literal kernel),
@@ -189,17 +213,18 @@ def roi_align_levels(feats, rois: torch.Tensor, output_size, spatial_scales: Seq
     staged = feats if isinstance(feats, StagedLevels) else None
     nl = len(feats)
     assert 1 <= nl <= L.MAX_LEVELS and len(spatial_scales) == nl
+    raw = staged.nchw if staged is not None else list(feats)
+    dtype = staged.dtype if staged is not None else _levels_dtype(raw)
     L.require_cuda(rois, "rois")
     assert rois.dim() == 2 and rois.size(1) == 5, "rois must have shape [K,5]"
-    raw = staged.nchw if staged is not None else list(feats)
     B, C = raw[0].shape[0], raw[0].shape[1]
     K = rois.size(0)
     dev = raw[0].device
     rois = rois.to(torch.float32).contiguous()
     if out is None:
-        out = torch.empty((K, C, ph, pw), dtype=torch.float32, device=dev)
+        out = torch.empty((K, C, ph, pw), dtype=dtype, device=dev)
     else:
-        assert out.shape == (K, C, ph, pw) and out.is_contiguous() and out.dtype == torch.float32
+        assert out.shape == (K, C, ph, pw) and out.is_contiguous() and out.dtype == dtype
     if K == 0:
         return out
     if bias is not None:
@@ -207,22 +232,28 @@ def roi_align_levels(feats, rois: torch.Tensor, output_size, spatial_scales: Seq
         bias = bias.contiguous()
     for f in raw:
         L.require_cuda(f, "feats")
-        assert f.dtype == torch.float32 and f.shape[0] == B and f.shape[1] == C
+        assert f.shape[0] == B and f.shape[1] == C
+    native = impl == "auto" and _fast_path_ok(C, ph, pw)
+    if dtype != torch.float32 and not native:
+        # no half-precision kernel for this shape / impl: the fp32 result, rounded once
+        res = roi_align_levels([f.float() for f in raw], rois, (ph, pw), spatial_scales, sampling_ratio, aligned, mode,
+                               finest_scale, impl, None, bias, pool2)
+        return out.copy_(res)
     Hs = (ctypes.c_int * nl)(*[int(f.shape[2]) for f in raw])
     Ws = (ctypes.c_int * nl)(*[int(f.shape[3]) for f in raw])
     sc = (ctypes.c_float * nl)(*[float(s) for s in spatial_scales])
     m = {"route": L.ROI_ROUTE, "sum": L.ROI_SUM}[mode]
     lib = L.lib()
-    if impl == "auto" and _fast_path_ok(C, ph, pw):
+    if native:
         bufs = staged.cg32 if staged is not None else [to_cg32(f) for f in raw]
         ptrs = (ctypes.c_void_p * nl)(*[b.data_ptr() for b in bufs])
         wsb = lib.nuhtc_roi_align_workspace_bytes(Hs, Ws, nl, B, K, ph, pw)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
         p2 = None if pool2 is None else (ctypes.c_int * nl)(*[int(bool(v)) for v in pool2])
         with torch.cuda.device(dev):
-            rc = lib.nuhtc_roi_align_cg32(ptrs, Hs, Ws, sc, nl, B, C, rois.data_ptr(), K, ph, pw, int(sampling_ratio),
-                                          int(bool(aligned)), m, float(finest_scale), p2, out.data_ptr(), L.ptr(bias), ws.data_ptr(),
-                                          wsb, L.stream_ptr(dev))
+            rc = lib.nuhtc_roi_align_cg32_dt(ptrs, Hs, Ws, sc, nl, B, C, rois.data_ptr(), K, ph, pw, int(sampling_ratio),
+                                             int(bool(aligned)), m, float(finest_scale), p2, out.data_ptr(), L.DTYPE_CODES[dtype],
+                                             L.ptr(bias), ws.data_ptr(), wsb, L.stream_ptr(dev))
         L.check(rc, "roi_align_cg32")
         L.count("roi_align_strip")
         if _RA_STATS:   # debugging aid (synchronises): how many RoIs missed the strip kernel

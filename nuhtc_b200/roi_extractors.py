@@ -6,6 +6,10 @@ multi-level RoIAlign launch (+ the fused attention pooling for AttentionRoIExtra
                                what the four shipped configs use)
 Both are plain ``nn.Module``s built from the same config dict (``roi_layer=dict(type='RoIAlign', output_size=..,
 sampling_ratio=..)``, ``out_channels``, ``featmap_strides``); inference only, GPU only.
+
+Precision: the reference's extractors are ``@force_fp32(apply_to=('feats',), out_fp16=True)``.  Here fp32, fp16 or bf16
+feats are all accepted and the RoI features come back in the feats' dtype, computed in fp32 and rounded once -- what
+force_fp32 does for fp16 once ``wrap_fp16_model`` has set ``fp16_enabled``, without its casts of the levels and results.
 """
 from __future__ import annotations
 
@@ -40,7 +44,7 @@ class _BaseRoIExtractor(nn.Module):
         self.roi_layers = nn.ModuleList([RoIAlign(spatial_scale=1 / s, **cfg) for s in featmap_strides])
         self.out_channels = out_channels
         self.featmap_strides = list(featmap_strides)
-        self.fp16_enabled = False
+        self.fp16_enabled = False   # set by mmcv's wrap_fp16_model; the output dtype follows the feats either way
 
     @property
     def num_inputs(self) -> int:
@@ -110,8 +114,8 @@ class AttentionRoIExtractor(_BaseRoIExtractor):
         bias: Optional[torch.Tensor] = None
         for i in attn:
             # the reference hard-codes the level stride as 4 * 2**i (roi_extractors_cus.py:222)
-            bias = attention_pool(feats[i], rois, 4 * 2 ** i, float(self.thres), out=bias)
+            bias = attention_pool(feats[i].float(), rois, 4 * 2 ** i, float(self.thres), out=bias)   # fp32 kernel, small levels
         if not pooled:
-            return bias[:, :, None, None].expand(-1, -1, *l0.output_size).contiguous()
+            return bias[:, :, None, None].expand(-1, -1, *l0.output_size).contiguous().to(feats[0].dtype)
         return roi_align_levels([feats[i] for i in pooled], rois, l0.output_size, [self.roi_layers[i].spatial_scale for i in pooled],
                                 l0.sampling_ratio, l0.aligned, mode="sum", bias=bias)

@@ -8,6 +8,10 @@ but keeps every intermediate on the GPU: no per-image Python loop, no ``.cpu().n
 and the paste, no per-instance D2H (SURVEY.md H7).  The ops are the ones in this package (one multi-level
 RoIAlign launch per cascade stage, one grouped NMS launch for all tiles, fused paste, batched mask NMS); the
 bbox / mask heads are callables supplied by the caller (stock PyTorch modules -- outside this package's target).
+
+Precision: the FPN levels (and the semantic feature map) may be fp32, fp16 or bf16.  The RoI features reach the heads in
+that dtype (see roi_align_levels), and the head outputs are upcast where mmdet's force_fp32 decorators upcast them:
+cls_score / bbox_pred before the activation and the box decode, the mask probabilities before the paste.
 """
 from __future__ import annotations
 
@@ -206,7 +210,7 @@ class RoIStage:
             bias = None
             for i in range(cfg.sum_levels, L_all):
                 # the reference hard-codes the level stride as 4 * 2**i (roi_extractors_cus.py:222)
-                bias = attention_pool(feats.nchw[i], rois, 4 * 2 ** i, float(cfg.attention_thres), out=bias)
+                bias = attention_pool(feats.nchw[i].float(), rois, 4 * 2 ** i, float(cfg.attention_thres), out=bias)
             lv = feats.sub(range(cfg.sum_levels))
             scales = [1.0 / s_ for s_ in cfg.featmap_strides[: cfg.sum_levels]]
             pool2 = [False] * cfg.sum_levels
@@ -234,9 +238,10 @@ class RoIStage:
     @torch.no_grad()
     def run(self, feats, rois: torch.Tensor, max_rois_per_tile: Optional[int] = None,
             semantic_feat: Optional[torch.Tensor] = None) -> RoIStageResult:
-        """feats: the FPN levels of the batch ([B,C,H_l,W_l] fp32 CUDA tensors) or an already staged ``StagedLevels``.
-        The kernel layout is staged ONCE here and handed to the four RoIAlign calls explicitly (no cache involved).
-        semantic_feat [B,C,H/stride,W/stride]: the semantic head's feature map (cfg.semantic_fusion)."""
+        """feats: the FPN levels of the batch ([B,C,H_l,W_l] fp32, fp16 or bf16 CUDA tensors) or an already staged
+        ``StagedLevels``.  The kernel layout is staged ONCE here and handed to the four RoIAlign calls explicitly (no cache
+        involved).  semantic_feat [B,C,H/stride,W/stride]: the semantic head's feature map (cfg.semantic_fusion), in the
+        levels' dtype."""
         cfg = self.cfg
         with self._t("stage_layout"):
             feats = stage_levels(feats)
@@ -256,12 +261,12 @@ class RoIStage:
             cls_score, bbox_pred = self.bbox_heads[i](bbox_feats)
             ms_scores.append(cls_score)
             if i < cfg.num_stages - 1:
-                # regress_by_class with reg_class_agnostic=True (mmdet bbox_head.py:459-496)
-                rois = det_ops.delta2bbox(rois, bbox_pred, stds=cfg.stage_stds[i], max_shape=cfg.img_shape)
-        cls_score = sum(ms_scores) / float(len(ms_scores))
-        scores = self.score_fn(cls_score)
+                # regress_by_class with reg_class_agnostic=True (mmdet bbox_head.py:459-496), force_fp32 on bbox_pred
+                rois = det_ops.delta2bbox(rois, bbox_pred.float(), stds=cfg.stage_stds[i], max_shape=cfg.img_shape)
+        cls_score = sum(ms_scores) / float(len(ms_scores))   # in the heads' dtype, as simple_test averages them
+        scores = self.score_fn(cls_score.float())           # get_bboxes is force_fp32 on cls_score / bbox_pred
         # rescale=True: detections live in the tile frame (bbox_head.py:373-376)
-        bboxes = det_ops.delta2bbox(rois, bbox_pred, stds=cfg.stage_stds[cfg.num_stages - 1], max_shape=cfg.img_shape,
+        bboxes = det_ops.delta2bbox(rois, bbox_pred.float(), stds=cfg.stage_stds[cfg.num_stages - 1], max_shape=cfg.img_shape,
                                     divide_by=cfg.scale_factor)[:, 1:]
 
         # multiclass_nms for every tile at once (nuhtc/models/bbox_head.py:12-102): class-agnostic boxes are
@@ -299,7 +304,7 @@ class RoIStage:
             mask_feats = self.extract(feats, mask_rois, cfg.mask_out, cfg.mask_sampling_ratio, sem, "mask")
         self._rec(mask_rois=mask_rois, mask_feats=mask_feats)
         logits = self.mask_head(mask_feats, det_cand)
-        probs = logits.sigmoid()
+        probs = logits.sigmoid().float()   # the paste works in fp32 (mmdet's _do_paste_mask casts the probabilities)
         H, W = cfg.ori_shape
         # the bit rows (+ area / tight box) feed the mask NMS; the dense uint8 frames are what get_seg_masks returns.
         # Both come straight from the 28x28 maps: re-reading 64 KB per nucleus to pack it would cost more than
