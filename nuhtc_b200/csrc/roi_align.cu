@@ -868,6 +868,9 @@ static int launch_pipe(const RoiLevels &lv, int B, int C, const float *rois, int
     static int grid_cache[kNuhtcMaxDevices] = {0};
     int &grid_cached = grid_cache[nuhtc_device()];
     static_assert(WMAX <= tmap_box_px(kTmapBoxes - 1) || true, "");
+    // the CTA's NQ * 4 channels must tile C: with C = 192 and 128-channel chunks, nchunk = 1 would read each pixel's
+    // 192 channels as 128 (NUHTC_RA_TMAP=2)
+    if (C % (NQ * 4) != 0) return 1; // caller falls back
     RoiTmaps tm;
     memset(&tm, 0, sizeof tm);
     if (C / (NQ * 4) > 1 && !cg32) {
@@ -1063,7 +1066,11 @@ static int roi_align_cg32_run(const RoiLevels &lv, int B, int C, const float *ro
                               int aligned, int mode, float finest_scale, OutT *out, int out_dtype, const float *bias, void *ws,
                               size_t ws_bytes, cudaStream_t st) {
     static const bool no_strip = getenv("NUHTC_RA_STRIP") && getenv("NUHTC_RA_STRIP")[0] == '0';   // A/B: per-RoI kernel only
-    if (roi_strip_supported(C, PH, PW, mode, lv.L) && !no_strip) {
+    // the strip prepass builds its tap tables at the output size: a pool2 level (a lone one in sum mode) needs the
+    // per-RoI kernels, which pool it with 2g samples per bin
+    bool pool2 = false;
+    for (int l = 0; l < lv.L; ++l) pool2 = pool2 || lv.pool2[l] != 0;
+    if (roi_strip_supported(C, PH, PW, mode, lv.L) && !no_strip && !pool2) {
         const int *left = nullptr, *left_count = nullptr;
         const int rc = roi_strip_forward(lv, B, C, rois, K, PH, sampling_ratio, aligned, mode, finest_scale, out, out_dtype, bias, ws,
                                          ws_bytes, st, &left, &left_count);
